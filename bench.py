@@ -31,6 +31,10 @@ step 0, which is what lets the same trials be checked against the CPU reference 
             source on the static tier; M/M/1 on the general engine), each timed
             the same way on this run's GPUs with its own parity sample against the reference build, and the
             single-core benchmark/MM1_single.c row.
+  --dump-outputs DIR
+            the per-trial results of the last timed step (what launch_trials returns: events, objects, t_end, sum_wait,
+            status, max_queue, counters) as DIR/<name>.npy in float64.  The same arguments give the same inputs on
+            every run, so two builds of the project can be compared output for output.
 """
 from __future__ import annotations
 
@@ -44,6 +48,7 @@ import time
 from pathlib import Path
 
 ROOT = Path(__file__).resolve().parent
+sys.dont_write_bytecode = True                 # the benchmark writes nothing into the tree it runs from
 sys.path.insert(0, str(ROOT))
 sys.path.insert(0, str(ROOT / "tests"))
 
@@ -69,7 +74,32 @@ def parse_args():
     p.add_argument("--no-secondary", action="store_true")
     p.add_argument("--single-process", action="store_true",
                    help="time cimba_b200_run_experiment_all_gpus (one host thread per GPU in THIS process) over --gpus GPUs")
+    p.add_argument("--dump-outputs", metavar="DIR",
+                   help="write the per-trial results of the last timed step to DIR/<name>.npy (float64)")
     return p.parse_args()
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(res, out_dir: str, rank: int, world: int) -> None:
+    """The arrays launch_trials hands its caller (TrialResults), as float64 .npy files, so that two builds can be
+    compared output for output.  Above DUMP_LIMIT_BYTES in all, a fixed seeded sample of trials is written, with
+    the trial indices beside it (trial_index.npy)."""
+    import numpy as np
+    arrays = {name: getattr(res, name).double().cpu().numpy()
+              for name in ("events", "objects", "t_end", "sum_wait", "status", "max_queue", "counters")}
+    n = len(arrays["events"])
+    per_trial = sum(a[0].nbytes for a in arrays.values())
+    if n * per_trial > DUMP_LIMIT_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(n, (DUMP_LIMIT_BYTES - 65536) // (per_trial + 8), replace=False))
+        arrays = {name: a[keep] for name, a in arrays.items()}
+        arrays["trial_index"] = keep.astype(np.float64)
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    suffix = f"_rank{rank}" if world > 1 else ""
+    for name, a in arrays.items():
+        np.save(out / f"{name}{suffix}.npy", a)
 
 
 # ------------------------------------------------------------------------------------------------ host facts
@@ -510,6 +540,8 @@ def main():
     kernel_ms = [a.elapsed_time(b) for a, b in per_launch]
     clocks = sampler.stop()
     diag_host = diag.cpu().tolist()
+    if args.dump_outputs:
+        dump_outputs(res, args.dump_outputs, rank, world)
 
     events_rank = int(res.events.sum().item())
     bad = int((res.status != 0).sum().item())

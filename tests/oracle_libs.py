@@ -5,10 +5,16 @@
 * ``load_ref()``   - oracle/_ref/librefdrv.so, model drivers linked against the
   unmodified reference library.  Present wherever `make -C oracle ref` has run
   (needs /root/reference); returns None otherwise.
+
+What the reference build returned for the runs the tests compare with is stored in
+tests/golden/reference_runs.json (tests/golden/make_reference_runs.py), so the
+comparisons hold wherever the suite runs.
 """
 from __future__ import annotations
 
 import ctypes as C
+import hashlib
+import json
 import subprocess
 from pathlib import Path
 
@@ -16,6 +22,24 @@ import numpy as np
 
 ROOT = Path(__file__).resolve().parents[1]
 ORACLE = ROOT / "oracle"
+REFERENCE_RUNS = ROOT / "tests/golden/reference_runs.json"
+
+
+def reference_runs():
+    return json.loads(REFERENCE_RUNS.read_text())
+
+
+def result_digest(rows):
+    """SHA-256 of result rows as tests/golden/reference_runs.json records them: one line per row, integers as unsigned
+    64-bit decimals, floating-point values (float32 widened exactly) as hex floats."""
+    text = "\n".join(" ".join(float(v).hex() if isinstance(v, (float, np.floating)) else str(int(v) & (2**64 - 1)) for v in row)
+                     for row in rows)
+    return hashlib.sha256(text.encode()).hexdigest()
+
+
+def trial_rows(results):
+    """run_trials results as digest rows: events, objects, t_end, sum_wait, max_fel, max_queue, the eight counters."""
+    return [(*r.key(), r.max_fel, r.max_queue, *r.counters()) for r in results]
 
 
 class Result(C.Structure):
@@ -141,6 +165,9 @@ class AwacsOut(C.Structure):
     def key(self):
         return (self.events, self.t_end, self.num_found, list(self.tds_count), list(self.mode_count),
                 self.sum_x, self.sum_y)
+
+    def row(self):
+        return (self.events, self.t_end, self.num_found, *self.tds_count, *self.mode_count, self.sum_x, self.sum_y)
 
 
 AWACS_TARGETS = 1000

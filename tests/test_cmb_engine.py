@@ -1,8 +1,8 @@
 """CPU tests of the general engine (cimba_b200/csrc/cmb_device.cuh) and of the models written against its authoring
 surface (cimba_b200/models/*.cuh, examples/tandem_model.cuh): the SAME source text compiled for the host
 (tests/cmb_engine_host.cpp) must reproduce, trial for trial, what the unmodified reference produced for the same
-models written against its own API (tests/golden/cmb_engine_vectors.json; and the live build oracle/_ref where
-present): event count, clock, sums, counters and the pop trace - M/M/1 (also in heavy traffic and overload, where the
+models written against its own API (tests/golden/cmb_engine_vectors.json, tests/golden/reference_runs.json): event
+count, clock, sums, counters and the pop trace - M/M/1 (also in heavy traffic and overload, where the
 queue grows without bound), G/G/1, M/M/c (3, 8 and 64 servers, overload), the reneging model with 40, 1000 and 1500
 processes (timers, cancels by handle, wait-list removals, the stop cascade) and the tandem model with a blocking put."""
 import ctypes as C
@@ -12,8 +12,10 @@ from pathlib import Path
 import pytest
 
 from cmb_cases import GOLD, MASTER, RESOURCEPOOL_GOLDEN_LINE, TRACE, case_id, check_trial, inverse_fmix64, wtdsummary_line
+from oracle_libs import reference_runs, result_digest
 
 ROOT = Path(__file__).resolve().parents[1]
+RUNS = reference_runs()
 
 
 class HostResult(C.Structure):
@@ -63,23 +65,18 @@ def test_engine_source_on_the_cpu_matches_the_reference_vectors(host, case):
             assert out[i].max_queue == want["max_fel"]          # the deepest the event list was at a pop
 
 
+def check_reference_run(host, case, counters):
+    """A case of tests/golden/reference_runs.json on the engine's host build: events, objects, t_end, sum_wait and the
+    first `counters` counters of every trial as the reference computed them."""
+    out, _, _ = run_host(host, case, case["count"], first=case["first"])
+    assert all(o.status == 0 for o in out), case
+    assert [o.events for o in out] == case["events"], case
+    assert result_digest([(o.events, o.objects, o.t_end, o.sum_wait, *list(o.counter)[:counters]) for o in out]) == case["sha256"], case
+
+
 def test_engine_matches_the_live_reference_build(host):
-    from oracle_libs import load_ref, run_trials
-    ref = load_ref()
-    if ref is None:
-        pytest.skip("oracle/_ref/librefdrv.so not built (needs /root/reference)")
-    ref.ref_set_param.argtypes = [C.c_int, C.c_double]
-    for model, servers, nobj, arr, srv, params in ((0, 1, 7000, 1.0, 1.0, []), (2, 5, 7000, 0.22, 1.0, []),
-                                                   (16, 300, 25, 2.5, 1.0, [0.9]), (17, 2, 7000, 1.2, 1.0, [])):
-        case = {"model": model, "servers": servers, "num_objects": nobj, "arr_mean": float(arr).hex(),
-                "srv_mean": float(srv).hex(), "params": params}
-        ref.ref_set_param(0, params[0] if params else 0.0)
-        want = run_trials(ref, "ref", model, servers, MASTER, 11, 5, nobj, arr, srv, par=0)
-        ref.ref_set_param(0, 0.0)
-        out, _, _ = run_host(host, case, 5, first=11)
-        for o, w in zip(out, want):
-            assert (o.events, o.objects, o.t_end, o.sum_wait) == (w.events, w.objects, w.t_end, w.sum_wait)
-            assert list(o.counter)[:4] == list(w.counter)[:4] or model != 16
+    for case in RUNS["engine_cases"]:
+        check_reference_run(host, case, 4)
 
 
 def test_a_small_arena_is_reported_not_survived_silently(host):
@@ -232,32 +229,9 @@ def test_static_tier_and_general_engine_agree_on_parameters_no_vector_covers(hos
 
 
 def test_engine_against_the_live_reference_on_drawn_parameters(host):
-    """Beyond the stored vectors: the reference's test worlds and tutorial 1 on the engine's host build against the live reference
-    build (oracle/_ref/librefdrv.so), parameters drawn here - capacities 1..40, durations, means, warm-up times."""
-    import random
-    from oracle_libs import load_ref, run_trials
-    ref = load_ref()
-    if ref is None:
-        pytest.skip("oracle/_ref/librefdrv.so not built (needs /root/reference)")
-    ref.ref_set_param.argtypes = [C.c_int, C.c_double]
-    rnd = random.Random(7)
-    try:
-        # (not model 18: its cmb_random_flip calls would leave cached bits in the reference's thread-local cache for later tests)
-        for model in (3, 4, 5, 6, 8, 9, 11, 12, 13, 14, 19):
-            for _ in range(3):
-                servers = 1 if model in (8, 9, 14, 19) else rnd.randint(1, 40)
-                nobj = rnd.randint(150, 1500)
-                arr, srv = rnd.choice([0.4, 0.7, 1.0, 1.6]), rnd.choice([0.6, 1.0, 1.4])
-                params = [rnd.uniform(0.0, 100.0)] if model == 19 else []
-                case = {"model": model, "servers": servers, "num_objects": nobj, "arr_mean": float(arr).hex(), "srv_mean": float(srv).hex(),
-                        "params": params}
-                first = rnd.randint(0, 5000)
-                ref.ref_set_param(0, params[0] if params else 0.0)
-                want = run_trials(ref, "ref", model, servers, MASTER, first, 4, nobj, arr, srv, par=0)
-                out, _, _ = run_host(host, case, 4, first=first)
-                for i, (o, w) in enumerate(zip(out, want)):
-                    assert o.status == 0, (case, i)
-                    assert (o.events, o.objects, o.t_end, o.sum_wait) == (w.events, w.objects, w.t_end, w.sum_wait), (case, i)
-                    assert list(o.counter) == list(w.counter), (case, i)
-    finally:
-        ref.ref_set_param(0, 0.0)
+    """Beyond the vectors of cmb_engine_vectors.json: the reference's test worlds and tutorial 1 on the engine's host build
+    against the reference's results on drawn parameters - capacities 1..40, durations, means, warm-up times
+    (tests/golden/make_reference_runs.py draws them), all eight counters."""
+    assert len(RUNS["engine_drawn_cases"]) == 33
+    for case in RUNS["engine_drawn_cases"]:
+        check_reference_run(host, case, 8)

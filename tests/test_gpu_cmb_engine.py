@@ -2,13 +2,12 @@
 
 * the models written against the authoring surface (M/M/1, G/G/1, M/M/c, the 1000-process reneging model) against the
   vectors the unmodified reference produced for the same models written against its own API
-  (tests/golden/cmb_engine_vectors.json) and, where it travelled with the snapshot, the live reference build;
+  (tests/golden/cmb_engine_vectors.json, tests/golden/reference_runs.json);
 * the repair pass: trials the fixed-capacity fast kernels flag (rho = 0.99, rho > 1, a wait list that outgrows its
   ring) come back with the reference's answer and a clean status word - the drop-in has no capacity the reference lacks;
 * MODEL_MMC with 64 servers (the fast kernel's event list holds 16 entries);
 * model libraries of one's own: examples/*.cu built with scripts/build_model.py, loaded with cimba_b200_model_load
   and run through cimba_b200_run_experiment like any built-in model."""
-import ctypes as C
 import sys
 from pathlib import Path
 
@@ -18,10 +17,11 @@ import torch
 
 import cimba_b200 as cb
 from cmb_cases import GOLD, MASTER, RESOURCEPOOL_GOLDEN_LINE, TRACE, case_id, check_trial, inverse_fmix64, wtdsummary_line
-from oracle_libs import load_port, load_ref, run_trials
+from oracle_libs import load_port, reference_runs, result_digest, run_trials
 
 pytestmark = pytest.mark.gpu
 ROOT = Path(__file__).resolve().parents[1]
+RUNS = reference_runs()
 BUILTIN = {0: cb.MODEL_MM1, 1: cb.MODEL_GG1, 2: cb.MODEL_MMC, 7: cb.MODEL_HOLD, 10: cb.MODEL_HARBOR, 16: cb.MODEL_RENEGE,
            18: cb.MODEL_POOL_RECORDED, 19: cb.MODEL_TUTORIAL1,
            # the reference's own test worlds: since round 2 they run on the general engine by default
@@ -133,20 +133,18 @@ def test_queue_capacities_the_round_one_tables_could_not_hold(model, servers):
 
 
 def test_reneging_model_against_the_live_reference_build():
-    ref = load_ref()
-    if ref is None:
-        pytest.skip("oracle/_ref/librefdrv.so did not travel with this snapshot")
-    ref.ref_set_param.argtypes = [C.c_int, C.c_double]
-    servers, think, srv, pat, T, n = 1200, 3.0, 1.0, 0.8, 30, 24
-    ref.ref_set_param(0, pat)
-    want = run_trials(ref, "ref", 16, servers, MASTER, 100, n, T, think, srv, par=1)
-    ref.ref_set_param(0, 0.0)
-    res = cb.run_trials(n, arr_mean=think, srv_mean=srv, num_objects=T, master_seed=MASTER, first_trial=100,
-                        model=cb.MODEL_RENEGE, servers=servers, params=[pat])
+    """1200 processes per trial: events, clock, sums and counters as the reference's pthread executive computed them
+    (tests/golden/reference_runs.json)."""
+    g = RUNS["renege"]
+    servers = g["servers"]
+    res = cb.run_trials(g["count"], arr_mean=float.fromhex(g["arr_mean"]), srv_mean=float.fromhex(g["srv_mean"]),
+                        num_objects=g["num_objects"], master_seed=MASTER, first_trial=g["first"], model=cb.MODEL_RENEGE,
+                        servers=servers, params=g["params"])
     assert res.status.abs().sum().item() == 0
     ev, te, sw, cnt = res.events.cpu().tolist(), res.t_end.cpu().tolist(), res.sum_wait.cpu().tolist(), res.counters.cpu().tolist()
-    for i, w in enumerate(want):
-        assert (ev[i], te[i], sw[i], cnt[i][:4]) == (w.events, w.t_end, w.sum_wait, list(w.counter)[:4]), i
+    assert ev == g["events"]
+    assert result_digest([(ev[i], te[i], sw[i], *cnt[i][:4]) for i in range(g["count"])]) == g["sha256"]
+    for i in range(g["count"]):
         assert cnt[i][6] == 1 and cnt[i][7] == servers          # the key map was in use; every process was created
 
 
@@ -223,35 +221,24 @@ def test_user_built_static_tier_libraries_match_the_reference():
 def test_tutorial_one_as_an_experiment_through_the_host_buffer_entry():
     """tutorial/tut_1_7.c: 39 utilisations x replications in ONE trial array, cimba_run_experiment over it, each trial's result
     the time-weighted mean queue length.  Here: the same array through cimba_b200_run_experiment (MODEL_TUTORIAL1, warm-up time in
-    the descriptor's params), every trial's avg_queue_length bit-identical to the unmodified reference running the tutorial's trial."""
-    ref = load_ref()
-    if ref is None:
-        pytest.skip("oracle/_ref/librefdrv.so did not travel with this snapshot")
-    ref.ref_set_param.argtypes = [C.c_int, C.c_double]
-    rhos = [0.025 * (k + 1) for k in range(39)]
-    reps, warmup, duration = 2, 100.0, 2000
+    the descriptor's params), every trial's avg_queue_length bit-identical to the unmodified reference running the tutorial's trial
+    (tests/golden/reference_runs.json: 39 utilisations x 2 replications, warm-up 100, 2000 time units)."""
+    g = RUNS["tutorial1"]
     dt = np.dtype([("arr_mean", "<f8"), ("srv_mean", "<f8"), ("events", "<u8"), ("t_end", "<f8"), ("status", "<u4"), ("pad", "<u4"),
                    ("counters", "<u8", (8,))])
-    exp = np.zeros(len(rhos) * reps, dtype=dt)
-    for i in range(len(exp)):
-        exp["arr_mean"][i], exp["srv_mean"][i] = 1.0 / rhos[i // reps], 1.0
-    cb.cimba_run_experiment(exp, model=cb.MODEL_TUTORIAL1, num_objects=duration, master_seed=MASTER, params=[warmup])
+    exp = np.zeros(len(g["arr_means"]), dtype=dt)
+    exp["arr_mean"], exp["srv_mean"] = [float.fromhex(a) for a in g["arr_means"]], 1.0
+    cb.cimba_run_experiment(exp, model=cb.MODEL_TUTORIAL1, num_objects=g["num_objects"], master_seed=MASTER, params=[g["warmup"]])
     assert not exp["status"].any()
-    ref.ref_set_param(0, warmup)
-    try:
-        for i in range(len(exp)):
-            w = run_trials(ref, "ref", 19, 1, MASTER, i, 1, duration, float(exp["arr_mean"][i]), 1.0, par=0)[0]
-            assert (int(exp["events"][i]), float(exp["t_end"][i])) == (w.events, w.t_end), i
-            assert [int(v) for v in exp["counters"][i]] == list(w.counter), i
-    finally:
-        ref.ref_set_param(0, 0.0)
+    assert [int(v) for v in exp["events"]] == g["events"]
+    assert result_digest([(exp["events"][i], exp["t_end"][i], *exp["counters"][i]) for i in range(len(exp))]) == g["sha256"]
     mean_len = exp["counters"][:, 3].copy().view("<f8")
     assert mean_len[-1] > mean_len[0]                   # rho 0.975 queues more than rho 0.025
 
 
 def test_theme_park_tutorial_on_device_matches_the_unmodified_tutorial_source():
     """MODEL_PARK = tutorial/tut_3_1.c on the general engine: 64 trials against the vectors of the unmodified tutorial source
-    (tests/golden/park_vectors.json), and 300 more against the tutorial itself where its build travelled with the snapshot."""
+    (tests/golden/park_vectors.json), and 300 more against the tutorial's results for them (tests/golden/reference_runs.json)."""
     import json
     gold = json.loads((ROOT / "tests/golden/park_vectors.json").read_text())
     n = len(gold["trials"])
@@ -261,24 +248,13 @@ def test_theme_park_tutorial_on_device_matches_the_unmodified_tutorial_source():
     for i, want in enumerate(gold["trials"]):
         means = [float(v).hex() for v in cnt[i][:5].copy().view("<f8")]
         assert (ev[i], float(te[i]).hex(), means) == (want["events"], want["t_end"], want["means"]), i
-    so = ROOT / "oracle/_ref/libtut3_ref.so"
-    ref = load_ref()
-    if ref is None or not so.exists():
-        return
-
-    class Tut3Out(C.Structure):
-        _fields_ = [("events", C.c_uint64), ("t_end", C.c_double), ("park", C.c_double), ("riding", C.c_double),
-                    ("waiting", C.c_double), ("walking", C.c_double), ("rides", C.c_double)]
-    lib = C.CDLL(str(so))
-    lib.tut3_ref_trial.argtypes = [C.c_uint64, C.POINTER(Tut3Out)]
-    first, more = 1000, 300
-    res = cb.run_trials(more, arr_mean=1.0, srv_mean=1.0, num_objects=0, master_seed=MASTER, first_trial=first, model=cb.MODEL_PARK)
+    g = RUNS["park"]
+    res = cb.run_trials(g["count"], arr_mean=1.0, srv_mean=1.0, num_objects=0, master_seed=MASTER, first_trial=g["first"],
+                        model=cb.MODEL_PARK)
+    assert res.status.abs().sum().item() == 0
     ev, te, cnt = res.events.cpu().tolist(), res.t_end.cpu().tolist(), res.counters.cpu().numpy()
-    for i in range(more):
-        o = Tut3Out()
-        assert lib.tut3_ref_trial(ref.ref_fmix64(MASTER, first + i), C.byref(o)) == 0
-        assert (ev[i], te[i]) == (o.events, o.t_end), i
-        assert list(cnt[i][:5].copy().view("<f8")) == [o.park, o.riding, o.waiting, o.walking, o.rides], i
+    assert ev == g["events"]
+    assert result_digest([(ev[i], te[i], *cnt[i][:5].copy().view("<f8")) for i in range(g["count"])]) == g["sha256"]
 
 
 def test_second_tutorial_on_device_matches_the_unmodified_tutorial_source():

@@ -1,7 +1,7 @@
 """CPU tests of the AWACS oracle (tutorial/tut_5_1.c, BASELINE config 5): the plain-C restatement
-(oracle/port/awacs_port.c) against the UNMODIFIED tutorial source compiled behind a stub hdf5.h
-(oracle/_ref/libawacs_ref.so) wherever that build is present, and against the vectors that build produced
-(tests/golden/awacs_vectors.json, tests/golden/make_golden.py --only-awacs) everywhere."""
+(oracle/port/awacs_port.c) against vectors the UNMODIFIED tutorial source compiled behind a stub hdf5.h
+(oracle/_ref/libawacs_ref.so) produced (tests/golden/awacs_vectors.json, tests/golden/make_golden.py --only-awacs;
+tests/golden/reference_runs.json, tests/golden/make_reference_runs.py)."""
 import ctypes as C
 import hashlib
 import json
@@ -10,9 +10,10 @@ from pathlib import Path
 import numpy as np
 import pytest
 
-from oracle_libs import (AWACS_TERRAIN_SEED, awacs_terrain, awacs_trial, load_awacs_ref, load_port)
+from oracle_libs import (AWACS_TERRAIN_SEED, awacs_terrain, awacs_trial, load_port, reference_runs, result_digest)
 
 GOLD = json.loads((Path(__file__).parent / "golden/awacs_vectors.json").read_text())
+RUNS = reference_runs()
 
 
 @pytest.fixture(scope="module")
@@ -59,33 +60,31 @@ def test_port_platform_state_matches_the_reference_vectors(port):
         assert [float(v).hex() for v in six] + [float(r.value).hex()] == want
 
 
-def test_port_matches_the_live_reference_build(port):
-    ref = load_awacs_ref()
-    if ref is None:
-        pytest.skip("oracle/_ref/libawacs_ref.so not built (needs /root/reference)")
-    rt = awacs_terrain(ref, "ref", 77, 8.0, 6.0)
-    pt = awacs_terrain(port, "port", 77, 8.0, 6.0)
-    assert rt[1:3] == pt[1:3] and np.array_equal(rt[3], pt[3])
-    assert np.array_equal(rt[0].view(np.uint32), pt[0].view(np.uint32))
-    for seed in (5, 6):
-        ro, rk, rtm, rper = awacs_trial(ref, "ref", seed, 0.03, trace_cap=3000)
-        po, pk, ptm, pper = awacs_trial(port, "port", seed, 0.03, pt, trace_cap=3000)
-        assert ro.key() == po.key() and rk == pk and rtm == ptm
-        assert rper["tds"] == pper["tds"] and rper["detected"] == pper["detected"] and rper["mode"] == pper["mode"]
-        assert np.array_equal(rper["x"].view(np.uint32), pper["x"].view(np.uint32))
+@pytest.fixture(scope="module")
+def small_terrain(port):
+    g = RUNS["awacs_terrain"]
+    return awacs_terrain(port, "port", g["seed"], g["width_nm"], g["height_nm"])
 
 
-def test_reference_executive_runs_awacs_trials_in_parallel(port):
-    """cimba_run_experiment over the tutorial's run_trial (all host cores) gives what one-at-a-time runs give."""
-    from oracle_libs import awacs_ref_experiment, load_ref
-    ref = load_awacs_ref()
-    if ref is None:
-        pytest.skip("oracle/_ref/libawacs_ref.so not built (needs /root/reference)")
-    pt = awacs_terrain(port, "port", 77, 8.0, 6.0)
-    awacs_terrain(ref, "ref", 77, 8.0, 6.0)
-    master = 0x34F05C64D7AD598F
-    outs = awacs_ref_experiment(ref, master, 3, 6, 0.02)
-    fmix = load_ref().ref_fmix64
-    for i, o in enumerate(outs):
-        po, _, _, _ = awacs_trial(port, "port", fmix(master, 3 + i), 0.02, pt)
-        assert o.key() == po.key()
+def test_port_matches_the_live_reference_build(port, small_terrain):
+    """A second terrain and two more trials (pop traces, every target's detect state, mode and position) as the
+    reference computed them (tests/golden/make_reference_runs.py)."""
+    m, cols, rows, geom = small_terrain
+    g = RUNS["awacs_terrain"]
+    assert (cols, rows) == (g["cols"], g["rows"]) and [float(v).hex() for v in geom] == g["geom"]
+    assert result_digest([m.view(np.uint32)]) == g["map_sha256"]
+    for want in RUNS["awacs_trials"]:
+        po, pk, ptm, pper = awacs_trial(port, "port", want["seed"], want["hours"], small_terrain, trace_cap=want["trace_cap"])
+        assert po.events == want["events"][0] and result_digest([po.row()]) == want["sha256"]
+        assert result_digest(zip(pk, ptm)) == want["trace_sha256"]
+        targets = zip(pper["tds"], pper["detected"], pper["mode"], pper["x"].view(np.uint32))
+        assert result_digest(targets) == want["targets_sha256"]
+
+
+def test_reference_executive_runs_awacs_trials_in_parallel(port, small_terrain):
+    """cimba_run_experiment over the tutorial's run_trial (all host cores) gave what one-at-a-time runs give when the
+    vectors were made; the port's trials give the same."""
+    g = RUNS["awacs_executive"]
+    outs = [awacs_trial(port, "port", port.port_fmix64(RUNS["master"], g["first"] + i), g["hours"], small_terrain)[0]
+            for i in range(g["count"])]
+    assert [o.events for o in outs] == g["events"] and result_digest([o.row() for o in outs]) == g["sha256"]

@@ -1,17 +1,18 @@
 """CPU tests: pin the plain-C oracle (oracle/port) to the reference.
 
-Two anchors: (1) the committed golden vectors generated from the unmodified
-reference build (tests/golden/make_golden.py), always; (2) the live reference
-build in oracle/_ref whenever it is present (build container), on more seeds.
+Two anchors, both generated from the unmodified reference build: (1) the golden
+vectors of tests/golden/make_golden.py; (2) the reference's results for more
+seeds and models (tests/golden/make_reference_runs.py).
 """
 import ctypes as C
 
 import numpy as np
 import pytest
 
-from oracle_libs import rng_draws, run_trials, trace_trial
+from oracle_libs import reference_runs, result_digest, rng_draws, run_trials, trace_trial, trial_rows
 
 KAT_SEED = 0x34F05C64D7AD598F
+RUNS = reference_runs()
 
 
 def _u64(a):
@@ -68,15 +69,13 @@ def test_remaining_distributions_match_golden(port, golden):
         assert int(np.add.reduce(u, dtype=np.uint64)) == g["sum"], tag
 
 
-def test_remaining_distributions_match_live_reference(port, ref):
+def test_remaining_distributions_match_live_reference(port):
+    """Kinds 9..33, two more seeds: every one of 8192 variates as the reference drew it."""
     from oracle_libs import DIST_CASES, rng_draws_ex
-    if ref is None:
-        pytest.skip("oracle/_ref not built here (no /root/reference)")
-    for kind, par in DIST_CASES:
-        for seed in (1, 0xC0FFEE):
-            a = rng_draws_ex(ref, "ref", seed, kind, par, 8192)
-            b = rng_draws_ex(port, "port", seed, kind, par, 8192)
-            assert a == b, (kind, par, seed)
+    assert [(g["kind"], g["params"]) for g in RUNS["distributions"][::2]] == [(k, list(p)) for k, p in DIST_CASES]
+    for g in RUNS["distributions"]:
+        b = rng_draws_ex(port, "port", g["seed"], g["kind"], g["params"], g["n"])
+        assert result_digest([(x,) for x in b]) == g["sha256"], (g["kind"], g["params"], g["seed"])
 
 
 def test_trials_match_golden(port, golden):
@@ -240,39 +239,25 @@ def test_heap_script_orders_like_the_comparator(port):
 
 # ------------------------------------------------------------------ live reference
 
-@pytest.mark.parametrize("model,arr,srv,servers", [(0, 1 / 0.9, 1.0, 1), (0, 1.25, 1.0, 1),
-                                                   (1, 1.25, 1.0, 1), (2, 1 / 6.4, 1.0, 8), (2, 0.5, 1.0, 3),
-                                                   (3, 1.0, 1.0, 10), (3, 0.5, 1.0, 2), (3, 0.7, 0.7, 1),
-                                                   (4, 1.0, 1.0, 20), (4, 1.0, 1.0, 5),
-                                                   (5, 1.0, 1.0, 10), (5, 0.5, 1.0, 2),
-                                                   (6, 1.0, 1.0, 8), (6, 0.5, 1.0, 2),
-                                                   (7, 1.0, 1.0, 500), (7, 0.5, 1.0, 5),
-                                                   (8, 1.0, 0.6, 1), (8, 0.4, 1.2, 1),
-                                                   (9, 1 / 0.9, 1.0, 1), (9, 2.0, 1.0, 1),
-                                                   (10, 2.0, 8.0, 10), (10, 1.2, 8.0, 4), (10, 0.9, 8.0, 3),
-                                                   (11, 1.0, 1.0, 10), (11, 0.5, 1.0, 2),
-                                                   (12, 1.0, 1.0, 10), (12, 0.5, 1.0, 4),
-                                                   (13, 1.0, 1.0, 10), (13, 0.5, 1.0, 3), (14, 1.0, 1.0, 1)])
-def test_port_equals_live_reference(port, ref, model, arr, srv, servers):
-    if ref is None:
-        pytest.skip("oracle/_ref not built here (no /root/reference)")
-    n = 48
-    size = 20_000 if model in (0, 1, 2, 9) else (30 if model == 7 else 1500)    # models 3..8: duration in time units
-    a = run_trials(ref, "ref", model, servers, 0xC0FFEE, 100, n, size, arr, srv, par=0)
-    b = run_trials(port, "port", model, servers, 0xC0FFEE, 100, n, size, arr, srv)
-    assert [x.key() for x in a] == [x.key() for x in b]
-    assert [(x.max_fel, x.max_queue) for x in a] == [(x.max_fel, x.max_queue) for x in b]
-    assert [x.counters() for x in a] == [x.counters() for x in b]
-    ra, ka, ta = trace_trial(ref, "ref", model, servers, 99, 3000 if model in (0, 1, 2, 9) else (15 if model == 7 else 800), arr, srv, 9000)
-    rb, kb, tb = trace_trial(port, "port", model, servers, 99, 3000 if model in (0, 1, 2, 9) else (15 if model == 7 else 800), arr, srv, 9000)
-    assert ka == kb and ta == tb and ra.key() == rb.key()
+@pytest.mark.parametrize("case", RUNS["port_cases"],
+                         ids=lambda c: f"{c['model']}-{c['arr']}-{c['srv']}-{c['servers']}")
+def test_port_equals_live_reference(port, case):
+    """48 trials per model and load (keys, max_fel / max_queue and counters) and one pop trace of up to 9000 pops,
+    as the reference computed them."""
+    model, servers, arr, srv = case["model"], case["servers"], case["arr"], case["srv"]
+    b = run_trials(port, "port", model, servers, case["master"], case["first"], case["count"], case["num_objects"], arr, srv)
+    assert [x.events for x in b] == case["events"]
+    assert result_digest(trial_rows(b)) == case["sha256"]
+    rb, kb, tb = trace_trial(port, "port", model, servers, case["trace_seed"], case["trace_objects"], arr, srv, case["trace_cap"])
+    assert result_digest([rb.key(), *zip(kb, tb)]) == case["trace_sha256"]
 
 
-def test_reference_pthread_executive_equals_serial(ref):
-    """cimba_run_experiment (all cores) vs the same trials run serially: the
-    multi-thread path the reference itself only smoke-tests (SURVEY.md section 4)."""
-    if ref is None:
-        pytest.skip("oracle/_ref not built here (no /root/reference)")
-    a = run_trials(ref, "ref", 0, 1, KAT_SEED, 0, 32, 5000, 1 / 0.9, 1.0, par=1)
-    b = run_trials(ref, "ref", 0, 1, KAT_SEED, 0, 32, 5000, 1 / 0.9, 1.0, par=0)
-    assert [x.key() for x in a] == [x.key() for x in b]
+def test_reference_pthread_executive_equals_serial(port):
+    """cimba_run_experiment (all cores) - the multi-thread path the reference itself only smoke-tests (SURVEY.md
+    section 4), checked against the same trials run serially when the vectors were made - against the port's trials,
+    serial and on its own pthread executive."""
+    g = RUNS["executive"]
+    for par in (0, 4):
+        b = run_trials(port, "port", g["model"], g["servers"], RUNS["master"], g["first"], g["count"], g["num_objects"],
+                       g["arr"], g["srv"], par=par)
+        assert result_digest([x.key() for x in b]) == g["sha256"]
