@@ -1638,7 +1638,12 @@ CMB_FN double draw_std_normal(Sim &sim) { return gp_std_normal(sim.rng, *sim.hot
 // cmb_process_hold(<a variate>) with the draw left to the dispatcher: the model's `double sample(S &sim, uint32_t id)` - a pure
 // function of the generator and the model's parameters, e.g. `return cmb_random_erlang(2u, 0.5 * arr_mean);` - is called right
 // after the body returns (same stream position as a draw in the hold's argument), where the warp is together; the static tier
-// first tries it with the ziggurats' hot paths only and parks the lane if that is not enough (cmb_static.cuh)
+// first tries it with the ziggurats' hot paths only and parks the lane if that is not enough (cmb_static.cuh).
+// The sampler may be any function that terminates on the reference with the same draws - a rejection loop included (an
+// exponential redrawn while above a cap, a normal redrawn while negative, a value only a ziggurat's tail can give): a try that
+// leaves the rectangles draws on - from the rectangles, and from a stand-in for the slow paths that reaches the same values -
+// until the sampler returns, and only then is thrown away and repeated.  It must not keep state across calls: it runs twice for
+// a hold whose first try missed the rectangles.
 #define CMB_PROCESS_HOLD_SAMPLED(id) \
     do { sim.cmd_sample = (id); sim.cmd = cimba_b200::cmb::CMD_HOLD_SAMPLED; CMB_YIELD_(); sig = sim.hold_end(me, sig); } while (0)
 // cmb_process_yield(): wait for whatever comes (a timer, a resume, an interrupt)

@@ -186,7 +186,7 @@ struct StaticSim {
     double         cmd_value;
     int64_t        cmd_exit;
     bool           hot_only;        // a sampler is being tried with the ziggurats' rectangles only ...
-    bool           hot_failed;      // ... and that was not enough: the draw will be repeated with the slow paths, in a batch
+    bool           hot_failed;      // ... and that was not enough: the try's result is void, the sampler is run again in a batch
     // where this trial's queues live: column `tid` of the CTA's shared-memory rings, and its HBM rings
     double        *ring_win;
     uint32_t       ring_stride;
@@ -314,17 +314,27 @@ struct StaticSim {
 
 // cmb_random_exponential / cmb_random_normal in a process body: inline (a call would take the generator's address and put the
 // whole control block in local memory)
-// In a sampler the dispatcher is trying out (hot_only), a draw that leaves its ziggurat's rectangles gives up - the dispatcher
-// rewinds the generator and repeats the whole sampler later, slow paths allowed, together with other lanes in the same position.
+// In a sampler the dispatcher is trying out (hot_only), a draw that leaves its ziggurat's rectangles marks the try as failed - the
+// dispatcher throws its result away, rewinds the generator and repeats the whole sampler later, slow paths allowed, together with
+// other lanes in the same position.  The failed try must still end: a sampler that redraws until it accepts (a truncated
+// exponential, a normal redrawn while negative, a value only a ziggurat's tail can give) loops forever on a constant it rejects.
+// So the generator keeps advancing, the rectangles still answer where they can, and where the slow path would run the try takes a
+// stand-in from the ziggurat's tail (its start plus an exponential): together they reach every value the reference's draw can, so
+// any sampler that ends on the reference ends here.  The stand-in is one out-of-line -log(u) of a raw output passed by value -
+// the slow paths themselves, inline at this call site as well, cost G/G/1 on the static tier a fifth of its throughput.
+CMB_FN_NOINLINE double stand_in_neg_log(uint64_t bits)
+{
+    return -log(__dmul_rn(__ull2double_rn((bits >> 11) + 1u), TWO_POW_M53));      // u in (0, 1]: finite
+}
+
 template <int NPROC, int NQUEUE, int NEVENT>
 CMB_FN double draw_exponential(StaticSim<NPROC, NQUEUE, NEVENT> &sim, double mean)        // include/cmb_random.h:319-352
 {
-    if (sim.hot_failed) return mean;
     const uint64_t u = sim.rng.next();
     if (Sfc64::exp_is_hot(u)) return __dmul_rn(mean, Sfc64::exp_hot(*sim.hot, u));
     if (sim.hot_only) {
         sim.hot_failed = true;
-        return mean;
+        return __dmul_rn(mean, __dadd_rn(ZIG_EXP_TAIL, stand_in_neg_log(sim.rng.next())));
     }
     return __dmul_rn(mean, sim.rng.exp_cold(u));
 }
@@ -332,13 +342,13 @@ CMB_FN double draw_exponential(StaticSim<NPROC, NQUEUE, NEVENT> &sim, double mea
 template <int NPROC, int NQUEUE, int NEVENT>
 CMB_FN double draw_std_normal(StaticSim<NPROC, NQUEUE, NEVENT> &sim)                       // include/cmb_random.h:206-215
 {
-    if (sim.hot_failed) return 1.0;
     const int64_t ix = (int64_t)sim.rng.next();
     const unsigned i = (unsigned)(ix & 0xff);
     if (i <= ZIG_NOR_MAX) return __dmul_rn(sim.hot->nor_x[i], __ll2double_rn(ix));
     if (sim.hot_only) {
         sim.hot_failed = true;
-        return 1.0;
+        const double x = __dadd_rn(ZIG_NOR_TAIL, __dmul_rn(ZIG_NOR_INV_TAIL, stand_in_neg_log(sim.rng.next())));
+        return ix < 0 ? -x : x;
     }
     return sim.rng.nor_cold(*sim.hot, ix);
 }

@@ -17,6 +17,12 @@
 //     shape < 1 (and what builds on it); geometric / negative_binomial apply ceil() to such a
 //     value and can differ by one on a measure-zero set.  glibc's log and pow tables were
 //     chosen by search and cannot be recomputed from first principles, so they stay CUDA's.
+// Where the reference itself is undefined, nothing can match it and nothing is promised:
+//   * geometric with p = 0, or with p so small that the count exceeds 2^32 (and negative_binomial / pascal on it): an
+//     out-of-range double converted to unsigned is undefined in C - x86 wraps, sm_100 saturates;
+//   * hyper-exponential and loaded dice whose probabilities sum to less than 1: the reference indexes past its table.
+// tests/test_random_edges.py and tests/test_gpu_random_edges.py hold every other edge (p = 0 and 1, lo == hi, a shape of
+// exactly 1, one degree of freedom, overflow to inf, subnormal results) to the reference's draws.
 // Compiled with -fmad=false: the expressions keep the reference's operation order.
 #pragma once
 

@@ -14,7 +14,8 @@
 // tail (recomputed here to 80 digits - it reproduces glibc's results, see below) and a degree-5 polynomial, the
 // multiply-adds fused as in glibc's x86-64 FMA build.  Checked on the CPU against glibc itself: 5e7 random
 // arguments in +-700, 0 mismatches (tests/test_awacs_math.py builds this same text for the host).
-// Arguments with |x| < 2^-54 or |x| >= 512 take the library exp() (never reached by the samplers).
+// glibc's special cases are restated too - |x| < 2^-54, |x| >= 1024, and 512 <= |x| < 1024 where the result nears overflow
+// or falls into the subnormal range (a lognormal reaches them) - so no argument takes the platform's own exp().
 #pragma once
 
 #include <cstdint>
@@ -99,14 +100,40 @@ static const uint64_t GLIBC_EXP_TAB[256] = {     // {tail bits, value bits - (i 
     0x3c77893b4d91cd9dull, 0x3fefe7c1819e90d8ull, 0x3c5305c14160cc89ull, 0x3feff3c22b8f71f1ull,
 };
 
+// glibc's specialcase(): a result near overflow, or in the subnormal range - rounded once there, as glibc does, not twice
+AW_MATH_FN double glibc_exp_specialcase(double tmp, uint64_t sbits, uint64_t ki)
+{
+    if ((ki & 0x80000000u) == 0u) {                     // k > 0: the scale's exponent may have overflowed by <= 460
+        const double scale = __longlong_as_double((long long)(sbits - (1009ull << 52)));
+        return __dmul_rn(0x1p1009, __fma_rn(scale, tmp, scale));
+    }
+    const double scale = __longlong_as_double((long long)(sbits + (1022ull << 52)));
+    const double st = __dmul_rn(scale, tmp);           // one product for both sums here: glibc's FMA build does not fuse them
+    double y = __dadd_rn(scale, st);
+    if (y < 1.0) {
+        double lo = __dadd_rn(__dsub_rn(scale, y), st);
+        const double hi = __dadd_rn(1.0, y);
+        lo = __dadd_rn(__dadd_rn(__dsub_rn(1.0, hi), y), lo);
+        y = __dsub_rn(__dadd_rn(hi, lo), 1.0);
+        if (y == 0.0) y = 0.0;
+    }
+    return __dmul_rn(0x1p-1022, y);
+}
+
 AW_MATH_FN double glibc_exp(double x)
 {
     const double InvLn2N = 0x1.71547652b82fep0 * 128, Shift = 0x1.8p52;
     const double NegLn2hiN = -0x1.62e42fefa0000p-8, NegLn2loN = -0x1.cf79abc9e3b3ap-47;
     const double C2 = 0x1.ffffffffffdbdp-2, C3 = 0x1.555555555543cp-3, C4 = 0x1.55555cf172b91p-5, C5 = 0x1.1111167a4d017p-7;
-    const uint32_t abstop = (uint32_t)((uint64_t)__double_as_longlong(x) >> 52) & 0x7ffu;
-    if (abstop - 0x3c9u >= 0x408u - 0x3c9u) {
-        return exp(x);
+    uint32_t abstop = (uint32_t)((uint64_t)__double_as_longlong(x) >> 52) & 0x7ffu;
+    if (abstop - 0x3c9u >= 0x408u - 0x3c9u) {            // |x| < 2^-54 or |x| >= 512: no libm call, so the device agrees too
+        if (abstop - 0x3c9u >= 0x80000000u) return __dadd_rn(1.0, x);
+        if (abstop >= 0x409u) {                          // |x| >= 1024, inf, NaN
+            if ((uint64_t)__double_as_longlong(x) == 0xfff0000000000000ull) return 0.0;
+            if (abstop >= 0x7ffu) return __dadd_rn(1.0, x);
+            return ((uint64_t)__double_as_longlong(x) >> 63) ? 0.0 : __longlong_as_double(0x7ff0000000000000ll);
+        }
+        abstop = 0u;                                     // 512 <= |x| < 1024: the scale may leave the exponent range
     }
     const double z = __dmul_rn(InvLn2N, x);
     double kd = __dadd_rn(z, Shift);
@@ -120,6 +147,7 @@ AW_MATH_FN double glibc_exp(double x)
     const double r2 = __dmul_rn(r, r);
     double tmp = __fma_rn(r2, __fma_rn(r, C3, C2), __dadd_rn(tail, r));
     tmp = __fma_rn(__dmul_rn(r2, r2), __fma_rn(r, C5, C4), tmp);
+    if (abstop == 0u) return glibc_exp_specialcase(tmp, sbits, ki);
     const double scale = __longlong_as_double((long long)sbits);
     return __fma_rn(scale, tmp, scale);
 }

@@ -23,7 +23,7 @@ int main(int argc, char **argv)
     const long n = argc > 1 ? std::atol(argv[1]) : 2000000;
     unsigned long bad = 0;
     for (long i = 0; i < n; i++) {
-        const double scale = (i & 3) == 0 ? 700.0 : ((i & 3) == 1 ? 40.0 : ((i & 3) == 2 ? 8.0 : 1.0e-3));
+        const double scale = (i & 3) == 0 ? 760.0 : ((i & 3) == 1 ? 40.0 : ((i & 3) == 2 ? 8.0 : 1.0e-3));
         const double x = (double)(int64_t)next64() / 9.3e18 * scale;
         const double a = std::exp(x), b = cimba_b200::glibc_exp(x);
         if (std::memcmp(&a, &b, 8) != 0) bad++;
